@@ -245,6 +245,17 @@ def recall_of(gt_ids, ids, counts):
     return hits / (ids.shape[0] * K)
 
 
+def dump_outputs(out_dir, ids, dists, counts, cmps, hops):
+    """--dump-outputs: the arrays one search step returns to its caller, as out_dir/<name>.npy, so that two builds
+    run with the same arguments (hence the same seeded inputs) can be compared output for output.  ids and the
+    per-query counters are uint32 and stored as float64 (exact); distances stay float32.  A step is at most
+    10K queries x k=10, about 1.4 MB in all."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("ids", ids), ("counts", counts), ("cmps", cmps), ("hops", hops)):
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a).view(np.uint32).astype(np.float64))
+    np.save(os.path.join(out_dir, "dists.npy"), np.ascontiguousarray(dists, np.float32))
+
+
 # ------------------------------------------------------------------------------------------ index preparation (GPU)
 
 def prepare_index(g, cfg, base, medoid, rank, world, dist, torch, log):
@@ -467,6 +478,8 @@ def run_gpu(args):
     step_no[0] = 0
     ms_dev_serial = timed(step_device, args.steps, args.warmup)
     launches = timed.launches
+    # the last step of the loop that `value` times: its buffers are overwritten by the loops and checks that follow
+    last_out = [t.cpu().numpy() for t in (d_ids, d_dists, d_counts, d_cmps, d_hops)] if args.dump_outputs else None
     step_no[0] = 0
     ms_e2e_serial = timed(step_e2e, args.steps, args.warmup)
     ms_dev, ms_e2e = ms_dev_serial, ms_e2e_serial
@@ -474,6 +487,9 @@ def run_gpu(args):
         step_no[0] = 0
         ms_dev = timed(step_device_async, args.steps, args.warmup, drain)
         launches = timed.launches
+        if args.dump_outputs:
+            o = sd[(args.warmup + args.steps - 1) % slots]
+            last_out = [o[f].cpu().numpy() for f in ("ids", "dists", "counts", "cmps", "hops")]
         step_no[0] = 0
         ms_e2e = timed(step_e2e_async, args.steps, args.warmup, drain)
     if args.profile_range:
@@ -581,6 +597,8 @@ def run_gpu(args):
         dist.barrier()
         dist.destroy_process_group()
     if rank == 0:
+        if args.dump_outputs:  # with several GPUs: rank 0's query shard
+            dump_outputs(args.dump_outputs, *last_out)
         emit(result)
 
 
@@ -754,6 +772,8 @@ def run_reference(args):
     cb = {"value": qps, "unit": "queries/s", "cores": threads, "kind": "port",
           "sample": f"each step = the first {m} queries of one of {NB} rotating 10K batches on {threads} threads (contiguous partitions)"}
     cb.update({k: hc[k] for k in ("cores_affinity", "cores_hw", "cgroup_cpu_quota", "cpu_model")})
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *outs[-1][1])
     emit({"impl": "reference", "metric": metric_name(cfg), "value": qps, "unit": "queries/s", "n_gpus": args.gpus,
           "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt * 1e3, "higher_is_better": True,
           "scaling": args.scaling, "vs_baseline": None, "dtype": cfg["dtype"], "data": "synthetic", "config": conf,
@@ -793,6 +813,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle parity gate (tuning runs only)")
     ap.add_argument("--profile-range", action="store_true", help="cudaProfilerStart/Stop around the timed region (for ncu)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the result arrays of the last one as DIR/<name>.npy")
     ap.add_argument("--prepare-only", default="", help=argparse.SUPPRESS)
     args = ap.parse_args()
     if args.warmup < 3:

@@ -5,6 +5,7 @@ import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -62,6 +63,42 @@ def test_reference_arm_prints_one_json_line_without_a_gpu():
     assert len(lines) == 1
     d = json.loads(lines[0])
     assert d["impl"] == "reference"
+
+
+def test_dump_outputs_stores_exact_float_arrays(tmp_path):
+    """ids and counters (uint32, the empty-slot id 0xFFFFFFFF included) round-trip exactly through float64."""
+    ids = np.array([[3, 0xFFFFFFFF], [0xFFFFFFFE, 7]], np.uint32)
+    dists = np.array([[0.5, np.inf], [1e-30, 2.0]], np.float32)
+    counters = np.array([1, 2], np.uint32)
+    bench.dump_outputs(str(tmp_path / "out"), ids.view(np.int32), dists, counters, counters + 10, counters + 20)
+    got = {f[:-4]: np.load(tmp_path / "out" / f) for f in os.listdir(tmp_path / "out")}
+    assert sorted(got) == ["cmps", "counts", "dists", "hops", "ids"]
+    assert got["dists"].dtype == np.float32 and np.array_equal(got["dists"].view(np.uint32), dists.view(np.uint32))
+    for name, want in (("ids", ids), ("counts", counters), ("cmps", counters + 10), ("hops", counters + 20)):
+        assert got[name].dtype == np.float64 and np.array_equal(got[name].astype(np.uint32), want), name
+
+
+@pytest.mark.gpu
+def test_bench_dumps_the_last_timed_step(tmp_path):
+    """--dump-outputs writes one search step's results (k sorted neighbours per query of the timed batch), and a second
+    run with the same arguments writes the same arrays."""
+    runs = []
+    for r in range(2):
+        out = tmp_path / f"run{r}"
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "small_100Kx128_f32_l2", "--steps", "5",
+                            "--warmup", "3", "--no-cpu-baseline", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, timeout=900)
+        assert p.returncode == 0, p.stderr[-2000:]
+        d = json.loads(p.stdout.strip().splitlines()[-1])
+        assert d["steps"] == 5 and d["config"]["parity_gate"]["result"] == "bit-identical"
+        runs.append({f: np.load(out / f"{f}.npy") for f in ("ids", "dists", "counts", "cmps", "hops")})
+    nq, n = d["config"]["queries_per_step"], d["config"]["n_points"]
+    a = runs[0]
+    assert a["ids"].shape == (nq, bench.K) and a["dists"].shape == (nq, bench.K) and a["counts"].shape == (nq,)
+    assert np.all(a["counts"] == bench.K) and np.all(a["ids"] < n) and np.all(np.diff(a["dists"], axis=1) >= 0)
+    assert np.all(a["cmps"] > 0) and np.all(a["hops"] > 0)
+    for f in a:
+        assert np.array_equal(a[f], runs[1][f]), f
 
 
 def test_traffic_json_is_keyed_by_workload(tmp_path, monkeypatch):
