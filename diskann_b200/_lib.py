@@ -8,7 +8,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("DAB_LIB_PATH") or os.path.join(_HERE, "libdiskann_b200.so")  # override: tuning builds
+LIB_PATH = os.environ.get("DAB_LIB_PATH") or os.path.join(_HERE, "libdiskann_b200.so")  # override: another build of the library (A/B)
 
 # every symbol include/diskann_b200.h declares: name -> (restype, argtypes)
 _vp, _u32, _u64, _i, _f = C.c_void_p, C.c_uint32, C.c_uint64, C.c_int, C.c_float
@@ -18,7 +18,6 @@ SYMBOLS = {
     "dab_last_error": (C.c_char_p, []),
     "dab_set_stream": (_i, [_vp, _vp]),
     "dab_launch_count": (_u64, []),
-    "dab_reload_tuning": (_i, [_vp]),
     "dab_upload_vectors": (_i, [_vp, _vp, _u64, _u64]),
     "dab_upload_vectors_device": (_i, [_vp, _vp, _u64, _u64]),
     "dab_upload_graph": (_i, [_vp, _vp, _u32, _u64, _u64]),

@@ -63,34 +63,11 @@ __global__ void repack_rows_kernel(const uint8_t* __restrict__ src, size_t src_s
     }
 }
 
-void Tuning::load() {
-    auto flag = [](const char* name) { return getenv(name) != nullptr; };
-    auto num = [](const char* name, long lo, long hi) -> int {
-        const char* t = getenv(name);
-        if (!t) return 0;
-        const long v = atol(t);
-        return v >= lo && v <= hi ? (int)v : 0;
-    };
-    disable_v2 = flag("DAB_DISABLE_V2");
-    disable_v3 = flag("DAB_DISABLE_V3");
-    v3_generic = flag("DAB_V3_GENERIC");
-    tc_resident = flag("DAB_TC_RESIDENT");
-    v3_max_cap = num("DAB_V3_MAX_CAP", 1, 512);
-    pq_ctas_per_sm = num("DAB_PQ_CTAS_PER_SM", 1, 16);
-    pq_global_lut = flag("DAB_PQ_GLOBAL_LUT");
-    pq_warps = num("DAB_PQ_WARPS", 1, 16);
-    pq_no_spec = flag("DAB_PQ_NO_SPEC");
-    pq_no_code_prefetch = flag("DAB_PQ_NO_CODE_PREFETCH");
-    frontier_narrow = flag("DAB_FRONTIER_NARROW");
-    v2_stage_bytes = num("DAB_V2_STAGE_BYTES", 1024, 65536);
-    v2_ctas_per_sm = num("DAB_V2_CTAS_PER_SM", 1, 64);
-    v2_slots = num("DAB_V2_SLOTS", 256, 1 << 24);
-    v2_full_grid = flag("DAB_V2_FULL_GRID");
-    v2_t1_bytes = getenv("DAB_V2_T1_BYTES") ? num("DAB_V2_T1_BYTES", 0, 64 * 1024) : -1;
-    v3_table_bytes = num("DAB_V3_TABLE_BYTES", 512, 200 * 1024);
-    v3_ctas_per_sm = num("DAB_V3_CTAS_PER_SM", 1, 32);
-    test_visited_log2 = num("DAB_TEST_VISITED_LOG2", 8, 30);
-    phase_profile = flag("DAB_PHASE_PROFILE");
+void TestHooks::load() {
+    const char* t = getenv("DAB_TEST_VISITED_LOG2");
+    const long v = t ? atol(t) : 0;
+    test_visited_log2 = v >= 8 && v <= 30 ? (int)v : 0;
+    pq_global_lut = getenv("DAB_TEST_PQ_GLOBAL_LUT") != nullptr;
 }
 
 }  // namespace dab
@@ -101,16 +78,6 @@ extern "C" {
 
 const char* dab_last_error(void) { return error_buffer(); }
 uint64_t dab_launch_count(void) { return g_launches.load(); }
-
-int dab_reload_tuning(dab_index* idx) {
-    if (!idx) return fail(DAB_ERR_INVALID_ARGUMENT, "dab_reload_tuning: idx is NULL");
-    idx->tune = Tuning();
-    idx->tune.load();
-    // what was learned under the previous settings (visited-set sizes per kernel) is forgotten
-    idx->hint_l = idx->hint_beam = idx->hint_visited = 0;
-    idx->pq_hint_l = idx->pq_hint_beam = idx->pq_hint_visited = 0;
-    return DAB_OK;
-}
 
 int dab_create(dab_index** out, int dtype, int metric, uint32_t dim, uint64_t n_points,
                uint32_t n_start, uint32_t max_degree, int device) {
@@ -142,7 +109,7 @@ int dab_create(dab_index** out, int dtype, int metric, uint32_t dim, uint64_t n_
     idx->adj_stride = (uint32_t)round_up((size_t)max_degree + 1, 8);
     idx->h_stage.pinned_host = true;
     idx->h_counters.pinned_host = true;
-    idx->tune.load();
+    idx->hooks.load();
     cudaError_t e = cudaStreamCreateWithFlags(&idx->own_stream, cudaStreamNonBlocking);
     if (e != cudaSuccess) {
         delete idx;
@@ -170,7 +137,6 @@ void dab_destroy(dab_index* idx) {
     search_slots_release(idx);
     comm_release(idx);
     tc_release(idx);
-    cudaFree(idx->d_phase_cycles);
     cudaFree(idx->d_vectors);
     cudaFree(idx->d_adj);
     cudaFree(idx->d_pivots);

@@ -57,28 +57,12 @@ struct Scratch {
     void release();
 };
 
-// Tuning / test knobs, read from the environment ONCE at dab_create (none changes results).
-struct Tuning {
-    bool disable_v2 = false;       // DAB_DISABLE_V2: skip search_kernel_v2
-    bool disable_v3 = false;       // DAB_DISABLE_V3: skip search_kernel_v3 (shared-memory visited sets)
-    bool frontier_narrow = false;  // DAB_FRONTIER_NARROW: 4-byte-load frontier kernel
-    int v2_stage_bytes = 0;        // DAB_V2_STAGE_BYTES
-    int v2_ctas_per_sm = 0;        // DAB_V2_CTAS_PER_SM
-    int v2_t1_bytes = -1;          // DAB_V2_T1_BYTES: shared-memory level of search_kernel_v2's visited set, bytes per warp (0: off; default 4096)
-    bool v2_full_grid = false;     // DAB_V2_FULL_GRID: launch every resident worker instead of balancing the rounds per worker
-    int v2_slots = 0;              // DAB_V2_SLOTS: cap on the visited-table slots per warp (smaller tables, more overflow re-runs)
-    int v3_table_bytes = 0;        // DAB_V3_TABLE_BYTES: visited-table bytes per warp
-    bool tc_resident = false;      // DAB_TC_RESIDENT: tensor-core scan keeps the query tile in shared memory (measured equal to streaming it)
-    int pq_ctas_per_sm = 0;        // DAB_PQ_CTAS_PER_SM: resident CTAs (4 warps) per SM of the PQ traversal kernel (default 6)
-    bool pq_global_lut = false;    // DAB_PQ_GLOBAL_LUT: PQ traversal with the per-warp table in global memory (search_kernel_pq) also where search_kernel_pqs fits
-    bool pq_no_spec = false;       // DAB_PQ_NO_SPEC: search_kernel_pqs without the adjacency row copied one hop ahead (L2 prefetch of the row only)
-    bool pq_no_code_prefetch = false;  // DAB_PQ_NO_CODE_PREFETCH: search_kernel_pqs without the L2 prefetch of probable candidates' codes
-    int pq_warps = 0;              // DAB_PQ_WARPS: cap on the warps (queries in flight) per CTA of search_kernel_pqs (default: what shared memory holds, <= 16)
-    int v3_max_cap = 0;            // DAB_V3_MAX_CAP: largest L + #start that still runs search_kernel_v3 (default 24)
-    bool v3_generic = false;       // DAB_V3_GENERIC: generic distance loop also for 32 / 64 / 96 / 128-d f32 rows
-    int v3_ctas_per_sm = 0;        // DAB_V3_CTAS_PER_SM: cap on resident CTAs
-    int test_visited_log2 = 0;     // DAB_TEST_VISITED_LOG2: tests force the overflow / retry path
-    bool phase_profile = false;    // DAB_PHASE_PROFILE: per-phase cycle sums of search_kernel_v2 (needs a -DDAB_PHASE_PROFILE_BUILD library)
+// Test hooks, read from the environment once at dab_create.  They let tests reach paths that small
+// inputs never select; none changes a result.
+struct TestHooks {
+    int test_visited_log2 = 0;  // DAB_TEST_VISITED_LOG2: visited tables small enough to take the overflow / re-run paths
+    bool pq_global_lut = false;  // DAB_TEST_PQ_GLOBAL_LUT: per-query PQ tables in global memory (search_kernel_pq MODE 0,
+                                 // pq_lut_kernel + pq_adc_kernel) even where they fit shared memory
     void load();
 };
 
@@ -125,7 +109,6 @@ struct dab_index {
     dab::Scratch h_stage;  // pinned host staging
     dab::Scratch h_counters;  // pinned: the four counters a search pass reports
     void* slots[DAB_MAX_SLOTS] = {};  // batches in flight (dab_search_batch_async), search_kernel.cu
-    unsigned long long* d_phase_cycles = nullptr;
 
     // search-side state learned across calls
     uint32_t hint_l = 0, hint_beam = 0, hint_visited = 0;  // largest visited set seen at (L, beam)
@@ -137,7 +120,7 @@ struct dab_index {
     cudaStream_t l2_window_stream = nullptr;
 
     uint64_t rec_truncated = 0;  // build: searches whose expanded-node record was cut at its capacity
-    dab::Tuning tune;
+    dab::TestHooks hooks;
 
     // tensor-core exhaustive scan (flat_tc.cu): bf16 operand copy of the rows + score coefficients
     void* d_tc_base = nullptr;

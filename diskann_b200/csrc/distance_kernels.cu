@@ -464,10 +464,8 @@ int launch_frontier(const dab_index* idx, const void* d_queries, uint32_t nq, co
     if (smem > 200 * 1024) return fail(DAB_ERR_INVALID_ARGUMENT, "dim %d too large for the frontier kernel", dim);
     cudaStream_t st = idx->stream;
     constexpr int U = 4;
-    // NA = 4 schemas over f32 / f16 rows: the wide-load kernel (16 B per lane)
-    const bool wide = plan.kind != KIND_COS && (idx->dtype == DAB_F32 || idx->dtype == DAB_F16) && idx->row_stride % 16 == 0 &&
-                      !idx->tune.frontier_narrow;  // DAB_FRONTIER_NARROW: tuning aid, forces the 4-byte-load kernel
-    if (wide) {
+    // NA = 4 schemas over f32 / f16 rows: the wide-load kernel (16 B per lane; rows start on 32 B bounds)
+    if (plan.kind != KIND_COS && (idx->dtype == DAB_F32 || idx->dtype == DAB_F16)) {
         const int qstride = (dim + 3) & ~3;
         const size_t wsmem = (size_t)kWarpsPerBlock * qstride * 4;
 #define LW(TQ, TDD, K, P)                                                                                          \
@@ -492,37 +490,16 @@ int launch_frontier(const dab_index* idx, const void* d_queries, uint32_t nq, co
         return DAB_OK;
     }
 #define ARGS nq, d_ids, c, idx->d_vectors, idx->row_stride, idx->n_total(), dim, d_out
+    // float cosine (NA = 2): the 4-byte-load kernel
     if (idx->dtype == DAB_F32) {
-#define L(K, P)                                                                                                   \
-    do {                                                                                                          \
-        if (K == KIND_COS) {                                                                                      \
-            auto kern = frontier_float_kernel<float, float, float, 2, K, P, U>;                                    \
-            cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                   \
-            kern<<<grid, block, smem, st>>>((const float*)d_queries, ARGS);                                       \
-        } else {                                                                                                  \
-            auto kern = frontier_float_kernel<float, float, float, 4, K, P, U>;                                    \
-            cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                   \
-            kern<<<grid, block, smem, st>>>((const float*)d_queries, ARGS);                                       \
-        }                                                                                                         \
-    } while (0)
-        DAB_KIND_POST_SWITCH(plan, L);
-#undef L
+        auto kern = frontier_float_kernel<float, float, float, 2, KIND_COS, POST_ONE_MINUS, U>;
+        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        kern<<<grid, block, smem, st>>>((const float*)d_queries, ARGS);
     } else if (idx->dtype == DAB_F16) {
-#define L(K, P)                                                                                                   \
-    do {                                                                                                          \
-        if (K == KIND_COS) {                                                                                      \
-            auto kern = frontier_float_kernel<float, __half, __half, 2, K, P, U>;                                  \
-            cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                   \
-            kern<<<grid, block, smem, st>>>((const __half*)d_queries, ARGS);                                      \
-        } else {                                                                                                  \
-            auto kern = frontier_float_kernel<float, __half, __half, 4, K, P, U>;                                  \
-            cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                   \
-            kern<<<grid, block, smem, st>>>((const __half*)d_queries, ARGS);                                      \
-        }                                                                                                         \
-    } while (0)
-        DAB_KIND_POST_SWITCH(plan, L);
-#undef L
-    } else if (is_int && dim % 16 == 0 && ((uintptr_t)d_queries & 15) == 0 && !idx->tune.frontier_narrow) {
+        auto kern = frontier_float_kernel<float, __half, __half, 2, KIND_COS, POST_ONE_MINUS, U>;
+        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        kern<<<grid, block, smem, st>>>((const __half*)d_queries, ARGS);
+    } else if (is_int && dim % 16 == 0 && ((uintptr_t)d_queries & 15) == 0) {
         const size_t ismem = (size_t)kWarpsPerBlock * dim;
 #define L(K, P)                                                                                   \
     do {                                                                                          \

@@ -37,9 +37,7 @@ int launch_frontier(const dab_index* idx, const void* d_queries, uint32_t nq, co
 namespace {
 
 constexpr int kBM = 128, kBN = 128, kBK = 64;  // CTA tile; one k-block = 64 bf16 = one 128-byte swizzle row
-constexpr int kStages = 5;                    // streaming mode: stages of (A k-block, B k-block)
-constexpr int kStagesRes = 4;                 // A-resident mode: stages of B k-blocks only
-constexpr int kMaxResKb = 6;                  // A stays in shared memory when K' <= 6 x 64 (e.g. 3 x 128)
+constexpr int kStages = 5;                    // stages of (A k-block, B k-block)
 constexpr int kTcThreads = 192;                // warp 0: TMA, warp 1: MMA + TMEM owner, warps 2-5: epilogue
 constexpr int kKP = 32;                        // largest candidate set per (query row, base range); k <= 10 uses 16
 constexpr uint32_t kTileBytes = kBM * kBK * 2; // 16 KB per operand tile
@@ -172,27 +170,23 @@ struct TcParams {
     uint32_t* cand;            // [nq][n_splits][kKP]
 };
 
-// RES: the 128 x K' query tile of the CTA is loaded once and stays in shared memory (K' <= 384), so only
-// base tiles stream from L2 — the operand traffic, which is what bounds this kernel, is halved.
-template <bool RES, int KP>
+template <int KP>
 __global__ void __launch_bounds__(kTcThreads, 1)
 flat_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, const TcParams p) {
-    constexpr int kSt = RES ? kStagesRes : kStages;
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    uint8_t* sa = smem;                                              // RES: kMaxResKb x 16 KB (whole A tile); else kStages x 16 KB
-    uint8_t* sb = smem + (RES ? kMaxResKb : kStages) * kTileBytes;   // kSt x 16 KB
-    float* s_coef = reinterpret_cast<float*>(sb + kSt * kTileBytes);  // [2 accumulators][alpha 128 | beta 128]
+    uint8_t* sa = smem;                                                   // kStages x 16 KB
+    uint8_t* sb = smem + kStages * kTileBytes;                            // kStages x 16 KB
+    float* s_coef = reinterpret_cast<float*>(sb + kStages * kTileBytes);  // [2 accumulators][alpha 128 | beta 128]
     float* s_scores = s_coef + 2 * 2 * kBN;                                      // [128 epilogue threads][33]: private scratch rows
     float* s_cd = s_scores + 128 * 33;                                           // [KP][128]: candidate scores, entry-major (conflict-free)
     uint32_t* s_ci = reinterpret_cast<uint32_t*>(s_cd + KP * 128);               // [KP][128]: candidate ids
     uint64_t* bars = reinterpret_cast<uint64_t*>(s_ci + KP * 128);               // offsets stay 8-byte aligned
-    uint64_t* full = bars;                  // [kSt] TMA -> MMA
-    uint64_t* empty = bars + kSt;           // [kSt] MMA -> TMA
-    uint64_t* tfull = bars + 2 * kSt;       // [2] MMA -> epilogue
-    uint64_t* tempty = tfull + 2;           // [2] epilogue -> MMA
-    uint64_t* afull = tempty + 2;           // [1] resident A tile has landed
-    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(afull + 1);
+    uint64_t* full = bars;                 // [kStages] TMA -> MMA
+    uint64_t* empty = bars + kStages;      // [kStages] MMA -> TMA
+    uint64_t* tfull = bars + 2 * kStages;  // [2] MMA -> epilogue
+    uint64_t* tempty = tfull + 2;          // [2] epilogue -> MMA
+    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(tempty + 2);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t m0 = blockIdx.y * kBM;
@@ -202,11 +196,10 @@ flat_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     const uint32_t kblocks = p.kp / kBK;
 
     if (threadIdx.x == 0) {
-        for (int s = 0; s < kSt; ++s) {
+        for (int s = 0; s < kStages; ++s) {
             mbar_init(full + s, 1);
             mbar_init(empty + s, 1);
         }
-        mbar_init(afull, 1);
         for (int a = 0; a < 2; ++a) {
             mbar_init(tfull + a, 1);
             mbar_init(tempty + a, 4);  // one arrival per epilogue warp
@@ -228,17 +221,13 @@ flat_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         // ===== TMA producer (one lane) =====
         if (lane == 0) {
             uint32_t stage = 0, phase = 0;
-            if (RES) {
-                mbar_expect_tx(afull, kblocks * kTileBytes);
-                for (uint32_t kb = 0; kb < kblocks; ++kb) tma_load_2d(&map_a, afull, sa + kb * kTileBytes, (int32_t)(kb * kBK), (int32_t)m0);
-            }
             for (uint32_t t = t0; t < t1; ++t) {
                 for (uint32_t kb = 0; kb < kblocks; ++kb) {
                     mbar_wait(empty + stage, phase ^ 1);
-                    mbar_expect_tx(full + stage, (RES ? 1 : 2) * kTileBytes);
-                    if (!RES) tma_load_2d(&map_a, full + stage, sa + stage * kTileBytes, (int32_t)(kb * kBK), (int32_t)m0);
+                    mbar_expect_tx(full + stage, 2 * kTileBytes);
+                    tma_load_2d(&map_a, full + stage, sa + stage * kTileBytes, (int32_t)(kb * kBK), (int32_t)m0);
                     tma_load_2d(&map_b, full + stage, sb + stage * kTileBytes, (int32_t)(kb * kBK), (int32_t)(t * kBN));
-                    if (++stage == kSt) {
+                    if (++stage == kStages) {
                         stage = 0;
                         phase ^= 1;
                     }
@@ -250,7 +239,6 @@ flat_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         if (lane == 0) {
             const uint32_t idesc = umma_idesc();
             uint32_t stage = 0, phase = 0;
-            if (RES) mbar_wait(afull, 0);
             for (uint32_t t = t0; t < t1; ++t) {
                 const uint32_t acc = (t - t0) & 1, use = (t - t0) >> 1;
                 mbar_wait(tempty + acc, (use & 1) ^ 1);  // the epilogue has drained this accumulator
@@ -261,12 +249,12 @@ flat_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 #pragma unroll
                     for (int k = 0; k < kBK / 16; ++k) {
-                        const uint64_t da = umma_desc(sa + (RES ? kb : stage) * kTileBytes, k * 32);
+                        const uint64_t da = umma_desc(sa + stage * kTileBytes, k * 32);
                         const uint64_t db = umma_desc(sb + stage * kTileBytes, k * 32);
                         umma_f16(tmem_d, da, db, idesc, (kb | (uint32_t)k) != 0 ? 1u : 0u);
                     }
                     umma_commit(empty + stage);  // frees the stage once these MMAs have read it
-                    if (++stage == kSt) {
+                    if (++stage == kStages) {
                         stage = 0;
                         phase ^= 1;
                     }
@@ -519,23 +507,15 @@ int dab_flat_knn_tc(dab_index* idx, const void* queries, uint32_t nq, uint32_t k
     p.alpha = (const float*)idx->d_tc_coef;
     p.beta = (const float*)idx->d_tc_coef + n;
     p.cand = (uint32_t*)idx->s_ids.p;
-    // resident query tile: halves the L2 -> SM operand traffic (12.4 -> 7.1 GB for 1000 x 1M), which bounds the
-    // kernel once the epilogue is out of the way (9.3 TB/s measured in streaming mode)
-    const bool resident = idx->tune.tc_resident && kp / kBK <= (uint32_t)kMaxResKb;
-    const size_t tiles_smem = resident ? (size_t)(kMaxResKb + kStagesRes) * kTileBytes : 2 * (size_t)kStages * kTileBytes;
-    const size_t smem = 1024 + tiles_smem + 2 * 2 * kBN * 4 + 128 * 33 * 4 + 2 * (size_t)kp_sel * 128 * 4 + (2 * (size_t)kStages + 5) * 8 + 16;
-#define DAB_TC_LAUNCH(RES_, KP_)                                                                                        \
-    do {                                                                                                                \
-        DAB_CUDA(cudaFuncSetAttribute(flat_tc_kernel<RES_, KP_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        flat_tc_kernel<RES_, KP_><<<dim3(splits, m_tiles), kTcThreads, smem, st>>>(map_a, map_b, p);                    \
+    const size_t tiles_smem = 2 * (size_t)kStages * kTileBytes;
+    const size_t smem = 1024 + tiles_smem + 2 * 2 * kBN * 4 + 128 * 33 * 4 + 2 * (size_t)kp_sel * 128 * 4 + (2 * (size_t)kStages + 4) * 8 + 16;
+#define DAB_TC_LAUNCH(KP_)                                                                                        \
+    do {                                                                                                          \
+        DAB_CUDA(cudaFuncSetAttribute(flat_tc_kernel<KP_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+        flat_tc_kernel<KP_><<<dim3(splits, m_tiles), kTcThreads, smem, st>>>(map_a, map_b, p);                    \
     } while (0)
-    if (resident) {
-        if (kp_sel == 16) DAB_TC_LAUNCH(true, 16);
-        else DAB_TC_LAUNCH(true, 32);
-    } else {
-        if (kp_sel == 16) DAB_TC_LAUNCH(false, 16);
-        else DAB_TC_LAUNCH(false, 32);
-    }
+    if (kp_sel == 16) DAB_TC_LAUNCH(16);
+    else DAB_TC_LAUNCH(32);
 #undef DAB_TC_LAUNCH
     DAB_LAUNCHED();
     DAB_CUDA(cudaGetLastError());

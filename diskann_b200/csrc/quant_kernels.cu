@@ -401,7 +401,7 @@ static bool fused_fits(const dab_index* idx, uint32_t* stride_out, size_t* piv_b
     *smem_out = piv_bytes + groups * group_floats * 4;
     if (groups_out) *groups_out = groups;
     if (group_floats_out) *group_floats_out = (uint32_t)group_floats;
-    return piv_bytes + group_floats * 4 <= 227 * 1024 && !idx->tune.pq_global_lut;
+    return piv_bytes + group_floats * 4 <= 227 * 1024 && !idx->hooks.pq_global_lut;
 }
 
 static int launch_fused(const dab_index* idx, const float* d_queries, uint32_t nq, int lut_metric, float* d_lut, const uint32_t* d_ids,

@@ -180,31 +180,15 @@ __device__ __forceinline__ void merge_any(float* qd, uint32_t* qi, uint32_t cap,
 // loads therefore carry the L2 evict_last priority (one 256-bit coherent load per bucket) and
 // the row copies evict_first (search_kernel_v2.cu), so the streaming rows do not push the
 // tables out of L2 and every probe is an L2 hit instead of a DRAM sector.
-#ifndef DAB_L2_HINTS
-#define DAB_L2_HINTS 1
-#endif
-
 __device__ __forceinline__ void load_bucket(const uint32_t* bp, uint32_t (&s)[8]) {
-#if DAB_L2_HINTS
     asm volatile("ld.relaxed.gpu.global.L2::evict_last.v8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
                  : "=r"(s[0]), "=r"(s[1]), "=r"(s[2]), "=r"(s[3]), "=r"(s[4]), "=r"(s[5]), "=r"(s[6]), "=r"(s[7])
                  : "l"(bp));
-#else
-    const uint4 lo = __ldcg(reinterpret_cast<const uint4*>(bp));
-    const uint4 hi = __ldcg(reinterpret_cast<const uint4*>(bp) + 1);
-    s[0] = lo.x, s[1] = lo.y, s[2] = lo.z, s[3] = lo.w, s[4] = hi.x, s[5] = hi.y, s[6] = hi.z, s[7] = hi.w;
-#endif
 }
 
 // table-clear store of one 32-byte bucket, same priority as the probes
 __device__ __forceinline__ void store_empty_bucket(uint32_t* bp) {
-#if DAB_L2_HINTS
     asm volatile("st.global.L2::evict_last.v8.b32 [%0], {%1,%1,%1,%1,%1,%1,%1,%1};" ::"l"(bp), "r"(kEmptyV2) : "memory");
-#else
-    const uint4 e4 = make_uint4(kEmptyV2, kEmptyV2, kEmptyV2, kEmptyV2);
-    reinterpret_cast<uint4*>(bp)[0] = e4;
-    reinterpret_cast<uint4*>(bp)[1] = e4;
-#endif
 }
 
 // One probe = one 32 B sector: returns true when `id` was newly inserted (HashSet::insert).

@@ -344,9 +344,6 @@ __global__ void __launch_bounds__(kSearchWarps * 32) search_kernel(const SearchP
 
 // ------------------------------------------------------------------ host side
 
-// search_kernel_v2.cu
-constexpr int kV2WarpsHost = kV2Warps;
-
 static uint32_t next_pow2_log2(uint64_t v) {
     uint32_t l = 0;
     while ((1ull << l) < v) ++l;
@@ -568,8 +565,7 @@ int SearchJob::prepare(const void* d_queries, const uint32_t* d_query_rows, uint
     }
     if (est > (double)idx->n_total() * 1.34) est = (double)idx->n_total() * 1.34;
     slots = std::max<uint64_t>(256, (uint64_t)est + 1);
-    if (idx->tune.test_visited_log2) slots = 1ull << idx->tune.test_visited_log2;  // tests force the overflow/retry path
-    if (idx->tune.v2_slots && use_v2 && slots > (uint64_t)idx->tune.v2_slots) slots = (uint64_t)idx->tune.v2_slots;
+    if (idx->hooks.test_visited_log2) slots = 1ull << idx->hooks.test_visited_log2;  // tests force the overflow/retry path
 
     if ((rc = counters->reserve(16 + (size_t)nq * 4))) return rc;
     d_counters = (uint32_t*)counters->p;
@@ -587,7 +583,7 @@ int SearchJob::prepare(const void* d_queries, const uint32_t* d_query_rows, uint
     pass = 0;
     uint32_t need = 0;
     if (hinted) need = (uint32_t)std::min<double>((double)idx->hint_visited * 1.15, 4.0e9);
-    if (idx->tune.test_visited_log2) need = (1u << idx->tune.test_visited_log2) / 2;
+    if (idx->hooks.test_visited_log2) need = (1u << idx->hooks.test_visited_log2) / 2;
     const bool skip = idx->v3_overflow_l == l_search && idx->v3_overflow_beam == beam && idx->v3_overflow_frac > 0.25f;
     memset(&p3, 0, sizeof(p3));
     if (!skip && v3_prepare(idx, l_search, beam, need, p3, v3) == 0) {
@@ -616,7 +612,7 @@ int SearchJob::launch() {
         v3.kern<<<launch_grid, kV3Warps * 32, v3.smem_block, stream>>>(p3);
     } else {
         // slots per warp: a power of two for the generic kernel, any multiple of 8 (32-byte buckets) for v2
-        const uint32_t warps = (uint32_t)grid * (use_v2 ? kV2WarpsHost : kSearchWarps);
+        const uint32_t warps = (uint32_t)grid * (use_v2 ? kV2Warps : kSearchWarps);
         const uint32_t hlog = std::max<uint32_t>(use_v2 ? 8 : 10, next_pow2_log2(slots));
         const uint32_t n_buckets = (uint32_t)((slots + 7) / 8);
         const size_t words_per_warp = use_v2 ? (size_t)n_buckets * 8 : ((size_t)1 << hlog);
@@ -629,22 +625,16 @@ int SearchJob::launch() {
             // one warp per query, persistent: size the grid so every resident warp runs the same
             // number of queries (10K queries on 3108 slots would otherwise pay for 4 full rounds
             // with the last one 22 % full)
-            const uint64_t max_warps = (uint64_t)grid * kV2WarpsHost;
+            const uint64_t max_warps = (uint64_t)grid * kV2Warps;
             const uint64_t rounds = (p.n_work + max_warps - 1) / max_warps;
             const uint64_t need = (p.n_work + rounds - 1) / rounds;
-            int launch_grid = (int)((need + kV2WarpsHost - 1) / kV2WarpsHost);
-            if (idx->tune.v2_full_grid || full_grid) launch_grid = (int)std::min<uint64_t>((uint64_t)grid, ((uint64_t)p.n_work + kV2WarpsHost - 1) / kV2WarpsHost);
-            p2.phase_cycles = nullptr;
-            if (idx->tune.phase_profile) {
-                if (!idx->d_phase_cycles) DAB_CUDA(cudaMalloc(&idx->d_phase_cycles, 64));
-                DAB_CUDA(cudaMemsetAsync(idx->d_phase_cycles, 0, 64, stream));
-                p2.phase_cycles = idx->d_phase_cycles;
-            }
+            int launch_grid = (int)((need + kV2Warps - 1) / kV2Warps);
+            if (full_grid) launch_grid = (int)std::min<uint64_t>((uint64_t)grid, ((uint64_t)p.n_work + kV2Warps - 1) / kV2Warps);
             p2.tables = p.tables;
             p2.n_buckets = n_buckets;
             p2.query_list = p.query_list;
             p2.n_work = p.n_work;
-            v2.kern<<<launch_grid, kV2WarpsHost * 32, v2.smem_block, stream>>>(p2);
+            v2.kern<<<launch_grid, kV2Warps * 32, v2.smem_block, stream>>>(p2);
         } else {
             const int launch_grid = (int)std::min<uint64_t>((uint64_t)grid, ((uint64_t)p.n_work + kSearchWarps - 1) / kSearchWarps);
             kern<<<launch_grid, kSearchWarps * 32, smem_block, stream>>>(p);
@@ -661,17 +651,6 @@ int SearchJob::finish() {
         DAB_CUDA(cudaStreamSynchronize(stream));
         idx->rec_truncated += h_counters[3];
         const uint32_t n_over = h_counters[1];
-        const uint32_t n_run = stage == 0 ? nq : p.n_work;
-        if (stage == 1 && use_v2 && p2.phase_cycles) {
-            unsigned long long h_ph[8];
-            DAB_CUDA(cudaMemcpy(h_ph, p2.phase_cycles, 64, cudaMemcpyDeviceToHost));
-            const char* names[8] = {"setup", "select", "adj+filter", "bulk-issue", "row-wait", "distance", "insert", "output"};
-            unsigned long long tot = 0;
-            for (int i = 0; i < 8; ++i) tot += h_ph[i];
-            fprintf(stderr, "[dab phase profile] nq=%u L=%u slots=%llu maxvisited=%u:", n_run, l_search, (unsigned long long)slots, h_counters[2]);
-            for (int i = 0; i < 8; ++i) fprintf(stderr, " %s=%.1f%%", names[i], tot ? 100.0 * h_ph[i] / tot : 0.0);
-            fprintf(stderr, " | cycles/query=%.0f\n", (double)tot / n_run);
-        }
         if (!recording) {  // build-time searches run on a growing graph: do not learn from them
             if (l_search != idx->hint_l || beam != idx->hint_beam) {
                 idx->hint_l = l_search;
@@ -703,7 +682,7 @@ int SearchJob::finish() {
             // the overflowed queries are the largest: size the global tables from the estimate again
             stage = 1;
             pass = 0;
-            if (!idx->tune.test_visited_log2)
+            if (!idx->hooks.test_visited_log2)
                 slots = std::max<uint64_t>(slots, std::min<uint64_t>((uint64_t)(1.1 * idx->max_degree * 1.3 * (double)l_search) + 1,
                                                                         (uint64_t)((double)idx->n_total() * 1.34) + 1));
         } else {

@@ -590,8 +590,6 @@ static int run_search_pq(dab_index* idx, const void* d_queries, uint32_t nq, uin
     if (use_pqs) {
         p.piv_stride = plan.piv_stride;
         p.piv_bytes = plan.piv_bytes;
-        p.spec_row = idx->tune.pq_no_spec ? 0 : 1;
-        p.code_prefetch = idx->tune.pq_no_code_prefetch ? 0 : 1;
         grid = plan.grid;
         warps = (uint32_t)plan.grid * (uint32_t)plan.warps;
     } else {
@@ -604,8 +602,8 @@ static int run_search_pq(dab_index* idx, const void* d_queries, uint32_t nq, uin
         if (per_sm < 1) return fail(DAB_ERR_INVALID_ARGUMENT, "dab_search_batch_pq: kernel does not fit");
         // every resident warp owns a LUT (n_chunks x n_centers f32: 32 KB at 32 x 256) and a visited table in
         // global memory; ADC terms and probes are L2 hits only while all of them stay L2-resident
-        // (the SQ kernel has no LUT: it keeps the occupancy the shared memory allows unless the knob is set)
-        if (mode == 0 || idx->tune.pq_ctas_per_sm) per_sm = std::min(per_sm, idx->tune.pq_ctas_per_sm ? idx->tune.pq_ctas_per_sm : 6);
+        // (the SQ kernel has no LUT: it keeps the occupancy the shared memory allows)
+        if (mode == 0) per_sm = std::min(per_sm, 6);
         grid = (int)std::min<uint64_t>((uint64_t)per_sm * idx->sm_count, ((uint64_t)nq + kPqWarps - 1) / kPqWarps);
         warps = (uint32_t)grid * kPqWarps;
     }
@@ -615,12 +613,12 @@ static int run_search_pq(dab_index* idx, const void* d_queries, uint32_t nq, uin
     // touches, and every query clears its table; queries that still overflow are re-run below
     uint64_t slots = std::max<uint64_t>(256, (uint64_t)(1.1 * idx->max_degree * 1.3 * (double)l_search) + 1);
     if (idx->pq_hint_visited > 0 && l_search <= idx->pq_hint_l && beam <= idx->pq_hint_beam && mode == idx->pq_hint_mode &&
-        !idx->tune.test_visited_log2) {
+        !idx->hooks.test_visited_log2) {
         const uint64_t seen = (uint64_t)(((double)idx->pq_hint_visited * 1.15 + idx->max_degree) / 0.875) + 8;
         slots = std::min(slots, std::max<uint64_t>(256, seen));
     }
     if (slots > 2 * idx->n_total() + 2048) slots = 2 * idx->n_total() + 2048;
-    if (idx->tune.test_visited_log2) slots = 1ull << idx->tune.test_visited_log2;  // tests force the overflow re-runs
+    if (idx->hooks.test_visited_log2) slots = 1ull << idx->hooks.test_visited_log2;  // tests force the overflow re-runs
     int rc;
     if ((rc = idx->s_counters.reserve(16 + (size_t)nq * 4))) return rc;
     uint32_t* d_counters = (uint32_t*)idx->s_counters.p;

@@ -57,8 +57,7 @@ __global__ void __launch_bounds__(kPqsMaxWarps * 32, 1) search_kernel_pqs(const 
     float* cd = reinterpret_cast<float*>(base + p.off_cd);
     uint32_t* beam_ids = reinterpret_cast<uint32_t*>(base + p.off_beam);
     uint32_t* nrow = reinterpret_cast<uint32_t*>(base + p.off_nrow);  // adjacency row copied one hop ahead (<= 96 words)
-    const bool spec_ok = p.adj_stride <= 96 && p.spec_row != 0;
-    const bool code_prefetch = p.code_prefetch != 0;
+    const bool spec_ok = p.adj_stride <= 96;
 
     const uint32_t warp_slot = blockIdx.x * (blockDim.x >> 5) + wib;
     const uint32_t nbk = p.n_buckets;
@@ -261,7 +260,7 @@ __global__ void __launch_bounds__(kPqsMaxWarps * 32, 1) search_kernel_pqs(const 
                                 }
                                 if (!found) {
                                     if (empty >= 0) {
-                                        if (code_prefetch && wd[t] < n_total) prefetch_l2(p.codes + (size_t)wd[t] * p.n_chunks);
+                                        if (wd[t] < n_total) prefetch_l2(p.codes + (size_t)wd[t] * p.n_chunks);
                                         old[t] = atomicCAS(table + (size_t)bk[t] * 8 + empty, kEmptyV2, wd[t]);
                                         state[t] = 1;
                                     } else {
@@ -358,7 +357,7 @@ __global__ void __launch_bounds__(kPqsMaxWarps * 32, 1) search_kernel_pqs(const 
 }
 
 bool pqs_plan(const dab_index* idx, uint32_t warp_smem, uint32_t nq, PqsPlan* out) {
-    if (idx->tune.pq_global_lut) return false;
+    if (idx->hooks.pq_global_lut) return false;
     if (idx->pq_chunks == 0 || idx->pq_chunks > 32) return false;  // a team of four lanes covers 32 chunks
     // pivot rows padded to an odd multiple of four floats: 16-byte aligned chunk loads, and the rows of eight
     // consecutive centres start in eight different 16-byte bank groups
@@ -367,7 +366,6 @@ bool pqs_plan(const dab_index* idx, uint32_t warp_smem, uint32_t nq, PqsPlan* ou
     const size_t piv_bytes = (size_t)idx->pq_centers * stride * 4;
     if (piv_bytes + 4 * (size_t)warp_smem > kPqsSmemLimit) return false;  // fewer than four warps would fit
     int warps = (int)std::min<size_t>(kPqsMaxWarps, (kPqsSmemLimit - piv_bytes) / warp_smem);
-    if (idx->tune.pq_warps) warps = std::min(warps, idx->tune.pq_warps);
     // small batches: spread the queries over the SMs instead of filling a few CTAs
     const int need = (int)(((uint64_t)nq + idx->sm_count - 1) / idx->sm_count);
     warps = std::max(std::min(warps, std::max(need, 4)), 1);

@@ -32,18 +32,8 @@
 namespace dab {
 
 constexpr int kGroup = 8;  // rows reduced together
-#ifndef DAB_V2_COPY8
-#define DAB_V2_COPY8 1     // row copies: eight lanes per row (0: whole warp per row)
-#endif
-#ifndef DAB_V2_ADJ_SMEM
-#define DAB_V2_ADJ_SMEM 1  // speculative adjacency row into shared memory (0: L2 prefetch)
-#endif
-#ifndef DAB_V2_INT_BUILD
-#define DAB_V2_INT_BUILD 1  // i8 / u8 rows in search_kernel_v2 (exact integer distances); GPU-validated in round 2
-#endif
-#ifndef DAB_V2_F32X2
-#define DAB_V2_F32X2 1     // packed FADD2 / FFMA2 distance arithmetic
-#endif
+// resident CTAs (one warp each) per SM the register budget is sized for
+constexpr int kV2MinCtas = 21;
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
@@ -87,7 +77,6 @@ __device__ __forceinline__ float group_distance(const float* __restrict__ q, con
                                                 uint32_t row_slot, int dim, int lane) {
     const int full8 = dim & ~7, rem = dim & 7;
     float v[kGroup];
-#if DAB_V2_F32X2
     uint64_t v2[kGroup / 2];
 #pragma unroll
     for (int g = 0; g < kGroup / 2; ++g) v2[g] = 0ull;
@@ -103,23 +92,6 @@ __device__ __forceinline__ float group_distance(const float* __restrict__ q, con
     }
 #pragma unroll
     for (int g = 0; g < kGroup / 2; ++g) unpack2(v2[g], v[2 * g], v[2 * g + 1]);
-#else
-#pragma unroll
-    for (int g = 0; g < kGroup; ++g) v[g] = 0.0f;
-    for (int e = lane; e < full8; e += 32) {
-        const float x = q[e];
-#pragma unroll
-        for (int g = 0; g < kGroup; ++g) {
-            const float y = to_f32(reinterpret_cast<const TD*>(rows + (size_t)g * row_slot)[e]);
-            if (KIND == KIND_L2) {
-                const float c = __fsub_rn(x, y);
-                v[g] = __fmaf_rn(c, c, v[g]);
-            } else {
-                v[g] = __fmaf_rn(x, y, v[g]);
-            }
-        }
-    }
-#endif
     bfly8<8>(v, lane, 8);
     bfly8<4>(v, lane, 16);
     if (rem) {
@@ -146,9 +118,7 @@ __device__ __forceinline__ float group_distance(const float* __restrict__ q, con
     return a;
 }
 
-
-#if DAB_V2_INT_BUILD
-// Experiment: i8 / u8 rows through the same hop structure.  Integer distances are exact in i32
+// i8 / u8 rows through the same hop structure.  Integer distances are exact in i32
 // (Sum(x-y)^2 = Sum x^2 + Sum y^2 - 2 Sum xy in wrapping arithmetic, as warp_int_multi), so any
 // summation order gives the reference's value: lane w owns 4-byte word w of all 8 staged rows.
 template <typename T>
@@ -204,7 +174,6 @@ __device__ __forceinline__ void group_distance_int(const uint8_t* __restrict__ q
         }
     }
 }
-#endif
 
 // Rare paths of the two-level visited set: clearing the warp's global table when its first id arrives, and the
 // atomic insert.  (The kernel is sensitive to its code size — at ~100 KB of SASS every phase ran ~20 % slower than at
@@ -228,10 +197,7 @@ __device__ __forceinline__ bool global_table_insert(uint32_t* table, uint32_t nb
 // so their visited set costs no global traffic at all; the global table is cleared when its first id arrives.
 // L1 = false: the global table alone (ids too wide for 14-bit tags at the table size, or level 1 disabled).
 template <typename TD, int KIND, int POST, int QT, bool L1>
-#ifndef DAB_V2_MIN_CTAS
-#define DAB_V2_MIN_CTAS 21
-#endif
-__global__ void __launch_bounds__(kV2Warps * 32, DAB_V2_MIN_CTAS) search_kernel_v2(const SearchParamsV2 p) {
+__global__ void __launch_bounds__(kV2Warps * 32, kV2MinCtas) search_kernel_v2(const SearchParamsV2 p) {
     extern __shared__ __align__(128) uint8_t smem[];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     uint8_t* base = smem + (size_t)wib * p.warp_smem;
@@ -256,12 +222,10 @@ __global__ void __launch_bounds__(kV2Warps * 32, DAB_V2_MIN_CTAS) search_kernel_
     const uint32_t hlimit = nbk * 7;  // 87.5 % load: 8-way buckets stay short
     const uint64_t n_total = p.n_points + p.n_start;
     const int dim = (int)p.dim;
-#if DAB_L2_HINTS
     // vector rows stream through L2 (a row is read once per query): evict them first so the
     // visited tables, which are re-probed every hop, stay resident
     uint64_t row_policy;
     asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(row_policy));
-#endif
 
     for (;;) {
         uint32_t w = 0;
@@ -270,33 +234,15 @@ __global__ void __launch_bounds__(kV2Warps * 32, DAB_V2_MIN_CTAS) search_kernel_
         if (w >= p.n_work) break;
         const uint32_t qidx = p.query_list ? p.query_list[w] : w;
 
-#ifdef DAB_PHASE_PROFILE_BUILD
-        long long tph[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-        long long tmark = clock64();
-#define DAB_PHASE(i)                         \
-    do {                                     \
-        if (p.phase_cycles) {                \
-            const long long _n = clock64();  \
-            tph[i] += _n - tmark;            \
-            tmark = _n;                      \
-        }                                    \
-    } while (0)
-#else
-#define DAB_PHASE(i) do { } while (0)
-#endif
-
         __syncwarp();
         {
             const TD* s = p.query_rows ? reinterpret_cast<const TD*>(p.vectors + (size_t)p.query_rows[qidx] * p.row_stride)
                                        : reinterpret_cast<const TD*>(p.queries) + (size_t)qidx * dim;
-#if DAB_V2_INT_BUILD
             if constexpr (V2Int<TD>::value) {
                 uint8_t* qb = reinterpret_cast<uint8_t*>(qf);
                 const int qbytes = (dim + 3) & ~3;
                 for (int e = lane; e < qbytes; e += 32) qb[e] = e < dim ? reinterpret_cast<const uint8_t*>(s)[e] : 0;
-            } else
-#endif
-            {
+            } else {
                 for (int e = lane; e < dim; e += 32) qf[e] = to_f32(s[e]);
             }
             if constexpr (L1) {
@@ -307,13 +253,10 @@ __global__ void __launch_bounds__(kV2Warps * 32, DAB_V2_MIN_CTAS) search_kernel_
             }
         }
         __syncwarp();
-#if DAB_V2_INT_BUILD
         int qq = 0;  // Sum x^2 of the query (unused by inner product)
         if constexpr (V2Int<TD>::value) {
             if (KIND != KIND_IP) qq = warp_int_self<V2Int<TD>::is_signed>(reinterpret_cast<const uint8_t*>(qf), dim, lane);
         }
-#endif
-        DAB_PHASE(0);  // query staging + table clear
 
         uint32_t size = 0, cursor_lo = 0, cmps = 0, hops = 0, nvisited = 0, nrec = 0;
         uint32_t n1 = 0;          // ids held by level 1 (nvisited counts those of the global table when L1 is on)
@@ -352,17 +295,9 @@ __global__ void __launch_bounds__(kV2Warps * 32, DAB_V2_MIN_CTAS) search_kernel_
         auto distances = [&](uint32_t c0, uint32_t n) {
             // eight lanes per row, 16 B each: one warp instruction moves 128 B of four different
             // rows, and every lane forms its own source address (no cross-lane traffic)
-#if DAB_V2_COPY8
             const uint32_t sub = (uint32_t)lane >> 3, nsub = 4, off0 = ((uint32_t)lane & 7u) * 16u, offs = 128;
-#else
-            const uint32_t sub = 0, nsub = 1, off0 = (uint32_t)lane * 16u, offs = 512;
-#endif
             auto copy16 = [&](uint32_t dst, const uint8_t* src) {
-#if DAB_L2_HINTS
                 asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "l"(row_policy) : "memory");
-#else
-                asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-#endif
             };
             // copies of rows [lo, hi) as one cp.async group
             auto issue = [&](uint32_t lo, uint32_t hi) {
@@ -383,7 +318,6 @@ __global__ void __launch_bounds__(kV2Warps * 32, DAB_V2_MIN_CTAS) search_kernel_
                 asm volatile("cp.async.commit_group;" ::: "memory");
             };
             auto compute = [&](uint32_t g0) {
-#if DAB_V2_INT_BUILD
                 if constexpr (V2Int<TD>::value) {
                     float vals[kGroup];
                     group_distance_int<V2Int<TD>::is_signed, KIND>(reinterpret_cast<const uint8_t*>(qf), rows + (size_t)g0 * p.row_slot,
@@ -391,19 +325,15 @@ __global__ void __launch_bounds__(kV2Warps * 32, DAB_V2_MIN_CTAS) search_kernel_
 #pragma unroll
                     for (int u = 0; u < kGroup; ++u)
                         if (lane == u && g0 + u < n) cd[c0 + g0 + u] = post_op<POST>(vals[u]);
-                } else
-#endif
-                {
+                } else {
                     const float r = group_distance<TD, KIND>(qf, rows + (size_t)g0 * p.row_slot, p.row_slot, dim, lane);
                     const uint32_t u = (((lane >> 3) & 1) << 2) | (((lane >> 4) & 1) << 1) | ((lane >> 2) & 1);
                     if ((lane & 3) == 0 && g0 + u < n) cd[c0 + g0 + u] = post_op<POST>(r);
                 }
             };
             issue(0, n);
-            DAB_PHASE(3);  // issue of the row copies
             asm volatile("cp.async.wait_group 0;" ::: "memory");
             __syncwarp();
-            DAB_PHASE(4);  // waiting for the rows
             for (uint32_t g0 = 0; g0 < n; g0 += kGroup) compute(g0);
             __syncwarp();
         };
@@ -453,7 +383,6 @@ __global__ void __launch_bounds__(kV2Warps * 32, DAB_V2_MIN_CTAS) search_kernel_
                 __syncwarp();
             }
             if (nb == 0) break;
-            DAB_PHASE(1);  // selection
 
             uint32_t ncand = 0;
             for (uint32_t b = 0; b < nb; ++b) {
@@ -560,17 +489,14 @@ __global__ void __launch_bounds__(kV2Warps * 32, DAB_V2_MIN_CTAS) search_kernel_
             }
             if (overflow) break;
             __syncwarp();
-            DAB_PHASE(2);  // adjacency fetch + visited filter
 
             for (uint32_t c0 = 0; c0 < ncand; c0 += p.stage_rows) distances(c0, min(p.stage_rows, ncand - c0));
-            DAB_PHASE(5);  // distance arithmetic
 
             // best.insert for every neighbour in adjacency order (index.rs:1986-1988)
             for (uint32_t c0 = 0; c0 < ncand; c0 += 32)
                 merge_round<QT>(qd, qi, p.cap, size, cursor_lo, cid, cd, c0, min(32u, ncand - c0), lane);
             cmps += ncand;
             hops += nb;
-            DAB_PHASE(6);  // inserts
         }
 
         if (overflow) {
@@ -613,12 +539,6 @@ __global__ void __launch_bounds__(kV2Warps * 32, DAB_V2_MIN_CTAS) search_kernel_
                 }
             }
         }
-        DAB_PHASE(7);  // output
-#ifdef DAB_PHASE_PROFILE_BUILD
-        if (p.phase_cycles && lane == 0)
-            for (int i = 0; i < 8; ++i) atomicAdd(p.phase_cycles + i, (unsigned long long)tph[i]);
-#endif
-#undef DAB_PHASE
     }
 }
 
@@ -626,16 +546,9 @@ __global__ void __launch_bounds__(kV2Warps * 32, DAB_V2_MIN_CTAS) search_kernel_
 // Returns 1 when this configuration is not covered by v2 (caller falls back to v1), 0 on
 // success with `out` filled, or a negative DAB error code.
 int v2_prepare(const dab_index* idx, uint32_t l_search, uint32_t beam, bool level1, SearchParamsV2& p, V2Launch& out) {
-    if (idx->tune.disable_v2) return 1;
-#if DAB_V2_INT_BUILD
     const bool v2_int = idx->dtype == DAB_I8 || idx->dtype == DAB_U8;
     const MetricPlan plan = plan_for(idx->metric, v2_int);
     if (plan.kind == KIND_COS && !v2_int) return 1;
-#else
-    if (idx->dtype != DAB_F32 && idx->dtype != DAB_F16) return 1;
-    const MetricPlan plan = plan_for(idx->metric, false);
-    if (plan.kind == KIND_COS) return 1;
-#endif
     const uint32_t cap = l_search + idx->n_start;
     if (cap > 256 || idx->max_degree > 1000) return 1;
     const uint32_t row_bytes = (uint32_t)round_up((size_t)idx->dim * elem_size(idx->dtype), 16);
@@ -643,11 +556,7 @@ int v2_prepare(const dab_index* idx, uint32_t l_search, uint32_t beam, bool leve
     const uint32_t row_slot = row_bytes;
     size_t off = 0;
     p.off_q = (uint32_t)off;
-#if DAB_V2_INT_BUILD
     off += v2_int ? round_up(round_up((size_t)idx->dim, 4), 16) : round_up((size_t)idx->dim * 4, 16);
-#else
-    off += round_up((size_t)idx->dim * 4, 16);
-#endif
     const size_t ncand_max = (size_t)beam * idx->max_degree;
     p.off_cid = (uint32_t)off;
     off += round_up(std::max<size_t>(ncand_max, idx->n_start) * 4, 16);
@@ -656,7 +565,7 @@ int v2_prepare(const dab_index* idx, uint32_t l_search, uint32_t beam, bool leve
     p.off_beam = (uint32_t)off;
     off += round_up((size_t)beam * 4, 16);
     // speculative adjacency buffer: the first <= 96 words of a row, 16-byte granules
-    p.adj_words = DAB_V2_ADJ_SMEM && idx->adj_stride % 4 == 0 ? (uint32_t)std::min<size_t>(idx->adj_stride, 96) : 0;
+    p.adj_words = idx->adj_stride % 4 == 0 ? (uint32_t)std::min<size_t>(idx->adj_stride, 96) : 0;
     p.off_adj = (uint32_t)off;
     off += (size_t)p.adj_words * 4;
     const size_t cap_pad = round_up(cap, 4);
@@ -668,8 +577,7 @@ int v2_prepare(const dab_index* idx, uint32_t l_search, uint32_t beam, bool leve
     p.off_rows = (uint32_t)off;
     const size_t fixed = off;
     // rows staged per round: as many as fit ~6 KB per warp, a multiple of the reduce group
-    size_t stage_bytes = 6144;
-    if (idx->tune.v2_stage_bytes) stage_bytes = (size_t)idx->tune.v2_stage_bytes;  // tuning aid
+    const size_t stage_bytes = 6144;
     uint32_t stage = (uint32_t)std::max<size_t>(kGroup, (stage_bytes / row_slot) / kGroup * kGroup);
     stage = std::min<uint32_t>(stage, 32);
     p.stage_rows = stage;
@@ -677,8 +585,7 @@ int v2_prepare(const dab_index* idx, uint32_t l_search, uint32_t beam, bool leve
     p.row_slot = row_slot;
     // level-1 visited table: 4 KB of 16-bit tags per warp (2048 slots; the mean visited set of the headline
     // workload is ~1200 ids) when the ids fit 14-bit quotient tags, i.e. n_total <= 16384 * buckets
-    size_t t1_bytes = idx->tune.v2_t1_bytes >= 0 ? (size_t)idx->tune.v2_t1_bytes : (idx->tune.test_visited_log2 ? 512 : 4096);  // tests: a level 1 that fills at once
-    t1_bytes = t1_bytes / 32 * 32;
+    size_t t1_bytes = idx->hooks.test_visited_log2 ? 512 : 4096;  // tests: a level 1 that fills at once
     p.t1_buckets = 0;
     if (t1_bytes >= 512) {
         uint32_t K = 8;
@@ -699,8 +606,8 @@ int v2_prepare(const dab_index* idx, uint32_t l_search, uint32_t beam, bool leve
     // the table traffic (8.8 -> 5.3 GB of DRAM traffic per 10K queries) and is 2 % faster, at C3 (12 -> 10) it is 11 % slower
     // ... and while batches overlap: one batch at a time is dominated by its tail, where the 4 resident warps fewer
     // cost more (2.96 vs 2.67 ms) than the traffic saves
-    if (p.t1_buckets && idx->tune.v2_t1_bytes < 0 && !level1) p.t1_buckets = 0;
-    if (p.t1_buckets && idx->tune.v2_t1_bytes < 0 && (227 * 1024) / (round_up((size_t)p.off_t1 + t1_bytes, 128) * kV2Warps + 1024) * kV2Warps < 16)
+    if (p.t1_buckets && !level1) p.t1_buckets = 0;
+    if (p.t1_buckets && (227 * 1024) / (round_up((size_t)p.off_t1 + t1_bytes, 128) * kV2Warps + 1024) * kV2Warps < 16)
         p.t1_buckets = 0;
     if (!p.t1_buckets) t1_bytes = 0;
     p.warp_smem = (uint32_t)round_up((size_t)p.off_t1 + t1_bytes, 128);
@@ -723,8 +630,7 @@ int v2_prepare(const dab_index* idx, uint32_t l_search, uint32_t beam, bool leve
         else if (plan.post == POST_NEG) PICK_Q(TD, KIND_IP, POST_NEG);    \
         else PICK_Q(TD, KIND_IP, POST_ONE_MINUS);                         \
     } while (0)
-#if DAB_V2_INT_BUILD
-#define PICK_I(TD)                                                       \
+#define PICK_I(TD)                                                     \
     do {                                                                 \
         if (plan.kind == KIND_L2) PICK_Q(TD, KIND_L2, POST_ID);           \
         else if (plan.kind == KIND_IP) PICK_Q(TD, KIND_IP, POST_NEG);     \
@@ -735,10 +641,6 @@ int v2_prepare(const dab_index* idx, uint32_t l_search, uint32_t beam, bool leve
     else if (idx->dtype == DAB_I8) PICK_I(int8_t);
     else PICK_I(uint8_t);
 #undef PICK_I
-#else
-    if (idx->dtype == DAB_F32) PICK_T(float);
-    else PICK_T(__half);
-#endif
 #undef PICK_T
 #undef PICK_Q
 #undef PICK2
@@ -751,7 +653,6 @@ int v2_prepare(const dab_index* idx, uint32_t l_search, uint32_t beam, bool leve
         cudaGetLastError();
         return 1;
     }
-    if (idx->tune.v2_ctas_per_sm && idx->tune.v2_ctas_per_sm < per_sm) per_sm = idx->tune.v2_ctas_per_sm;  // tuning aid
     out.grid = per_sm * idx->sm_count;
     return 0;
 }

@@ -35,28 +35,17 @@ namespace dab {
 
 namespace {
 
-#ifndef DAB_V3_LP16
-#define DAB_V3_LP16 0  // visited set: 1 = linear-probing 16-bit slots (measured slower: dependent probe steps), 0 = buckets of 16 tags
-#endif
-#ifndef DAB_V3_FAST_ONE
-#define DAB_V3_FAST_ONE 1  // fast f32 path: one 4-row pass per step (measured best: 2.71 vs 2.90 ms on C2); 0: two passes + butterfly
-#endif
-
 // ---- f32 rows of 32 * nm <= 128 elements (the headline shapes: 128-d, 96-d) ------------------
 // Same lane mapping and association as wide_distances, with the per-hop overheads removed: the
-// 16 query elements a lane ever multiplies live in registers (packed pairs), a step covers 8
-// rows (two passes) whose 8 x nm 16-byte loads are issued back to back, and the two passes are
-// reduced together with a transpose-butterfly — 9 shuffles + 9 adds for 8 rows instead of 24 +
-// 30: stage A (xor 2) adds accumulator pairs while splitting the passes between the lanes,
-// stage B (xor 4) finishes (s0+s1)+(s2+s3) while splitting the slots, stage C (xor 1) is
-// x_i + x_{i+4}, then (t0+t2) and (t1+t3) (xor 4) and their sum (xor 1).
+// 16 query elements a lane ever multiplies live in registers (packed pairs), and a step covers 4
+// rows (one pass, 8 lanes per row) whose nm 16-byte loads per lane are issued back to back.  The
+// reduction is xor 2 and xor 4 for (s0+s1)+(s2+s3), xor 1 for x_i + x_{i+4}, then (t0+t2)+(t1+t3).
 template <int KIND, int POST>
 __device__ __forceinline__ void wide_distances_f32_fast(const uint64_t (&q2)[8], int nm, const uint8_t* __restrict__ vectors,
                                                         size_t row_stride, const uint32_t* __restrict__ cid, uint32_t n,
                                                         float* __restrict__ cd, int lane) {
     const int team = lane >> 3, tl = lane & 7;
-#if DAB_V3_FAST_ONE
-    // one pass (4 rows) per step: 16 fewer registers, for the 5-CTA (20 warps per SM) build
+    // one pass per step measured faster than two passes reduced by a butterfly (2.71 vs 2.90 ms on C2)
     if (n > 4) prefetch_rows(vectors, row_stride, cid, n, (uint32_t)nm * 128u, lane);
     for (uint32_t j0 = 0; j0 < n; j0 += 4) {
         const uint8_t* row0 = vectors + (size_t)cid[min(j0 + team, n - 1)] * row_stride + 16 * tl;
@@ -86,50 +75,6 @@ __device__ __forceinline__ void wide_distances_f32_fast(const uint64_t (&q2)[8],
         const float r = __fadd_rn(__fadd_rn(ts[0], ts[2]), __fadd_rn(ts[1], ts[3]));
         if (tl == 0 && j0 + team < n) cd[j0 + team] = post_op<POST>(r);
     }
-    return;
-#endif
-    const bool pA = (tl & 2) != 0, pB = (tl & 4) != 0, hh = (tl & 1) != 0;
-    if (n > 8) prefetch_rows(vectors, row_stride, cid, n, (uint32_t)nm * 128u, lane);
-    for (uint32_t j0 = 0; j0 < n; j0 += 8) {
-        const bool two = j0 + 4 < n;  // warp-uniform: the second pass has rows
-        const uint8_t* row0 = vectors + (size_t)cid[min(j0 + team, n - 1)] * row_stride + 16 * tl;
-        const uint8_t* row1 = vectors + (size_t)cid[min(j0 + 4 + team, n - 1)] * row_stride + 16 * tl;
-        uint4 v0[4], v1[4];
-#pragma unroll
-        for (int m = 0; m < 4; ++m) {
-            if (m < nm) {
-                v0[m] = ldg16(row0 + m * 128);
-                if (two) v1[m] = ldg16(row1 + m * 128);
-            }
-        }
-        uint64_t a0[2] = {0ull, 0ull}, a1[2] = {0ull, 0ull};
-#pragma unroll
-        for (int m = 0; m < 4; ++m) {
-            if (m < nm) {
-                a0[0] = step2<KIND>(a0[0], q2[2 * m], pack2(__uint_as_float(v0[m].x), __uint_as_float(v0[m].y)));
-                a0[1] = step2<KIND>(a0[1], q2[2 * m + 1], pack2(__uint_as_float(v0[m].z), __uint_as_float(v0[m].w)));
-                if (two) {
-                    a1[0] = step2<KIND>(a1[0], q2[2 * m], pack2(__uint_as_float(v1[m].x), __uint_as_float(v1[m].y)));
-                    a1[1] = step2<KIND>(a1[1], q2[2 * m + 1], pack2(__uint_as_float(v1[m].z), __uint_as_float(v1[m].w)));
-                }
-            }
-        }
-        float x0[4], x1[4];
-        unpack2(a0[0], x0[0], x0[1]);
-        unpack2(a0[1], x0[2], x0[3]);
-        unpack2(a1[0], x1[0], x1[1]);
-        unpack2(a1[1], x1[2], x1[3]);
-        float v[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) v[i] = __fadd_rn(pA ? x1[i] : x0[i], __shfl_xor_sync(kFull, pA ? x0[i] : x1[i], 2));
-        const float w0 = __fadd_rn(pB ? v[2] : v[0], __shfl_xor_sync(kFull, pB ? v[0] : v[2], 4));
-        const float w1 = __fadd_rn(pB ? v[3] : v[1], __shfl_xor_sync(kFull, pB ? v[1] : v[3], 4));
-        const float u = __fadd_rn(hh ? w1 : w0, __shfl_xor_sync(kFull, hh ? w0 : w1, 1));  // x_i + x_{i+4}, i = 2 pB + h
-        const float z = __fadd_rn(u, __shfl_xor_sync(kFull, u, 4));                        // t0 + t2 | t1 + t3
-        const float r = __fadd_rn(z, __shfl_xor_sync(kFull, z, 1));
-        const uint32_t jj = j0 + (pA ? 4 : 0) + team;  // lanes with pA hold the second pass
-        if ((tl == 0 || tl == 2) && jj < n) cd[jj] = post_op<POST>(r);
-    }
 }
 
 template <typename T>
@@ -137,26 +82,16 @@ struct IsInt {
     static constexpr bool value = std::is_same<T, int8_t>::value || std::is_same<T, uint8_t>::value;
 };
 
-#ifndef DAB_V3_MIN_CTAS
-#define DAB_V3_MIN_CTAS 4
-#endif
-#ifndef DAB_V3_P_F32
-#define DAB_V3_P_F32 2  // f32 rows: passes (of 4 rows, 4 x 16-byte loads per lane each) in flight
-#endif
-#ifndef DAB_V3_P_F16
-#define DAB_V3_P_F16 2  // f16 rows: passes (of 8 rows) in flight
-#endif
-#ifndef DAB_V3_U_F16
-#define DAB_V3_U_F16 4  // f16 rows: 16-byte loads per lane per pass in flight
-#endif
-#ifndef DAB_V3_P_INT
-#define DAB_V3_P_INT 4  // i8 / u8 rows: passes (of 4 rows, one 16-byte load per lane each) in flight
-#endif
+constexpr int kV3MinCtas = 4;  // resident CTAs per SM the register budget is sized for
+constexpr int kV3PassesF32 = 2;  // f32 rows: passes (of 4 rows, 4 x 16-byte loads per lane each) in flight
+constexpr int kV3PassesF16 = 2;  // f16 rows: passes (of 8 rows) in flight
+constexpr int kV3LoadsF16 = 4;   // f16 rows: 16-byte loads per lane per pass in flight
+constexpr int kV3PassesInt = 4;  // i8 / u8 rows: passes (of 4 rows, one 16-byte load per lane each) in flight
 
 }  // namespace
 
 template <typename TD, int KIND, int POST, int QT, bool FAST>
-__global__ void __launch_bounds__(kV3Warps * 32, DAB_V3_MIN_CTAS) search_kernel_v3(const SearchParamsV3 p) {
+__global__ void __launch_bounds__(kV3Warps * 32, kV3MinCtas) search_kernel_v3(const SearchParamsV3 p) {
     extern __shared__ __align__(128) uint8_t smem[];
     constexpr bool kInt = IsInt<TD>::value;
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -171,19 +106,11 @@ __global__ void __launch_bounds__(kV3Warps * 32, DAB_V3_MIN_CTAS) search_kernel_
     const uint32_t adjbuf_a = smem_addr(adjbuf);
     uint32_t* table = reinterpret_cast<uint32_t*>(base + p.off_table);
     const uint32_t nbk = p.n_buckets;
-#if DAB_V3_LP16
-    const Lp16Map tmap{p.tag_kmask, nbk * 16, p.tag_magic, p.tag_shift, p.tag_bits, p.tag_dmax};
-#else
     const Tag16Map tmap{p.tag_kmask, nbk, p.tag_magic, p.tag_shift};
-#endif
     auto visit = [&](uint32_t id, bool& ovf) -> bool {
-#if DAB_V3_LP16
-        return lp16_insert(table, tmap, id, ovf);
-#else
         uint32_t bk, tg;
         tag16_of(id, tmap, bk, tg);
         return smem16_insert(table, nbk, bk, tg, ovf);
-#endif
     };
     const uint64_t n_total = p.n_points + p.n_start;
     const int dim = (int)p.dim;
@@ -236,14 +163,14 @@ __global__ void __launch_bounds__(kV3Warps * 32, DAB_V3_MIN_CTAS) search_kernel_
 
         auto distances = [&](uint32_t c0, uint32_t n) {
             if constexpr (kInt) {
-                wide_distances_int<std::is_same<TD, int8_t>::value, KIND, POST, DAB_V3_P_INT>(reinterpret_cast<const uint8_t*>(qf), qq, p.vectors,
+                wide_distances_int<std::is_same<TD, int8_t>::value, KIND, POST, kV3PassesInt>(reinterpret_cast<const uint8_t*>(qf), qq, p.vectors,
                                                                                  p.row_stride, cid + c0, n, cd + c0, dim, lane);
             } else if constexpr (sizeof(TD) == 2) {
-                wide_distances<TD, KIND, POST, DAB_V3_P_F16, DAB_V3_U_F16>(qf, p.vectors, p.row_stride, cid + c0, n, cd + c0, dim, lane);
+                wide_distances<TD, KIND, POST, kV3PassesF16, kV3LoadsF16>(qf, p.vectors, p.row_stride, cid + c0, n, cd + c0, dim, lane);
             } else if constexpr (FAST) {
                 wide_distances_f32_fast<KIND, POST>(q2, (int)p.fast_nm, p.vectors, p.row_stride, cid + c0, n, cd + c0, lane);
             } else {
-                wide_distances<TD, KIND, POST, DAB_V3_P_F32, 4>(qf, p.vectors, p.row_stride, cid + c0, n, cd + c0, dim, lane);
+                wide_distances<TD, KIND, POST, kV3PassesF32, 4>(qf, p.vectors, p.row_stride, cid + c0, n, cd + c0, dim, lane);
             }
             __syncwarp();
         };
@@ -412,11 +339,10 @@ __global__ void __launch_bounds__(kV3Warps * 32, DAB_V3_MIN_CTAS) search_kernel_
 
 // ------------------------------------------------------------------ host side
 int v3_prepare(const dab_index* idx, uint32_t l_search, uint32_t beam, uint32_t visited_need, SearchParamsV3& p, V3Launch& out) {
-    if (idx->tune.disable_v3) return 1;
     // v3 wins for short candidate lists (C2: 1.11 vs 1.67 ms at L = 15) and loses at the headline L = 100
     // (2.94 vs 2.68 ms); the measured crossover is L ~ 25 on both the 128-d f32 and the 768-d f16 shape
     // (profiles/r02_sweep_l.txt): longer lists go to the global-table kernel
-    if (l_search + idx->n_start > (uint32_t)(idx->tune.v3_max_cap ? idx->tune.v3_max_cap : 24)) return 1;
+    if (l_search + idx->n_start > 24) return 1;
     const bool is_int = idx->dtype == DAB_I8 || idx->dtype == DAB_U8;
     const MetricPlan plan = plan_for(idx->metric, is_int);
     if (plan.kind == KIND_COS && !is_int) return 1;  // float cosine: NA = 2 schema, generic kernel
@@ -456,33 +382,11 @@ int v3_prepare(const dab_index* idx, uint32_t l_search, uint32_t beam, uint32_t 
         const long long per_cta = (long long)(smem_sm / ctas) - 1024;
         return (per_cta / kV3Warps - (long long)fixed) / 32 * 32;
     };
-    // registers bound the residency (DAB_V3_MIN_CTAS CTAs per SM), so the table takes all the shared
+    // registers bound the residency (kV3MinCtas CTAs per SM), so the table takes all the shared
     // memory that residency leaves: a smaller table would only overflow more often
-    long long tbytes = table_bytes_at(DAB_V3_MIN_CTAS);
-    if (idx->tune.test_visited_log2 && visited_need)  // tests: a table small enough to overflow
+    long long tbytes = table_bytes_at(kV3MinCtas);
+    if (idx->hooks.test_visited_log2 && visited_need)  // tests: a table small enough to overflow
         tbytes = (long long)round_up((size_t)((visited_need + idx->max_degree) / 0.875) * 2 + 32, 32);
-    if (idx->tune.v3_table_bytes > 0) tbytes = (long long)round_up((size_t)idx->tune.v3_table_bytes, 32);
-#if DAB_V3_LP16
-    if (tbytes < 1024) tbytes = 1024;
-    if (tbytes > table_bytes_at(1)) return 1;
-    const uint64_t nbk = (uint64_t)tbytes / 32;
-    const uint64_t n_slots = nbk * 16;
-    uint32_t sbits = 0;
-    while (((uint64_t)1 << sbits) < n_slots) ++sbits;
-    // magic = ceil(2^(K+s) / n_slots) < 2^(K+1) fits 32 bits and h * magic < 2^(2K+1) fits 64 for K <= 30
-    const uint64_t tag_max = ((((uint64_t)1 << K) - 1)) / n_slots;
-    uint32_t tag_bits = 0;
-    while (((uint64_t)1 << tag_bits) <= tag_max) ++tag_bits;
-    if (tag_bits > 10) return 1;  // fewer than 6 displacement bits: index too large for this table size
-    p.n_buckets = (uint32_t)nbk;
-    p.tag_kmask = (uint32_t)(((uint64_t)1 << K) - 1);
-    p.tag_shift = K + sbits;
-    p.tag_magic = (uint32_t)((((uint64_t)1 << (K + sbits)) + n_slots - 1) / n_slots);
-    p.tag_bits = tag_bits;
-    p.tag_dmax = (1u << (16 - tag_bits)) - 2;
-    p.visited_limit = (uint32_t)(n_slots * 7 / 8);
-    (void)min_buckets;
-#else
     if (tbytes < (long long)min_buckets * 32) tbytes = (long long)min_buckets * 32;
     if (tbytes > table_bytes_at(1)) return 1;
     uint64_t nbk = (uint64_t)tbytes / 32;
@@ -494,8 +398,7 @@ int v3_prepare(const dab_index* idx, uint32_t l_search, uint32_t beam, uint32_t 
     p.tag_shift = K + sbits;
     p.tag_magic = (uint32_t)((((uint64_t)1 << (K + sbits)) + nbk - 1) / nbk);
     p.visited_limit = (uint32_t)(nbk * 14);  // 87.5 % of 16 tags per bucket
-#endif
-    p.fast_nm = (idx->dtype == DAB_F32 && idx->dim % 32 == 0 && idx->dim <= 128 && !idx->tune.v3_generic) ? idx->dim / 32 : 0;
+    p.fast_nm = (idx->dtype == DAB_F32 && idx->dim % 32 == 0 && idx->dim <= 128) ? idx->dim / 32 : 0;
     out.capacity = p.visited_limit > idx->max_degree ? p.visited_limit - idx->max_degree : 0;
     if (out.capacity < 4 * idx->max_degree) return 1;
     p.warp_smem = (uint32_t)round_up(fixed + (size_t)tbytes, 128);
@@ -540,7 +443,6 @@ int v3_prepare(const dab_index* idx, uint32_t l_search, uint32_t beam, uint32_t 
         cudaGetLastError();
         return 1;
     }
-    if (idx->tune.v3_ctas_per_sm && idx->tune.v3_ctas_per_sm < per_sm) per_sm = idx->tune.v3_ctas_per_sm;  // tuning aid
     out.grid = per_sm * idx->sm_count;
     return 0;
 }

@@ -52,8 +52,6 @@ struct SearchParamsPq {
     // search_kernel_pqs: the pivot table of the CTA in shared memory
     uint32_t piv_stride;  // floats between pivot rows (odd multiple of 4: rows of different centres start in different 16-byte bank groups)
     uint32_t piv_bytes;   // n_centers * piv_stride * 4, the per-warp slices follow
-    int spec_row;         // copy the probable next node's adjacency row one hop ahead + prefetch its buckets
-    int code_prefetch;    // L2 prefetch of the codes of probable new candidates before their inserts resolve
 };
 
 // search_kernel_pqs.cu — the shape of one launch of the shared-memory-pivot kernel

@@ -61,50 +61,6 @@ __device__ __forceinline__ bool smem16_insert(uint32_t* table, uint32_t n_bucket
     }
 }
 
-// ---- linear-probing variant: one 16-bit entry per slot ---------------------------------------
-// id -> h = (id * odd) mod 2^K (a bijection), home slot = h mod n_slots, tag = h div n_slots.
-// An entry stores (displacement << tag_bits) | tag, so an entry found d slots after its home
-// is unambiguous; entries are never removed, hence everything between an id's home and its
-// slot stays occupied and a lookup can stop at the first empty slot.  0xFFFF marks empty.
-// One probe step is one 32-bit shared-memory load and two compares (against ~90 instructions for
-// a 16-entry bucket scan); at the load the search runs at (<= 87 %, typically 30 %) a probe
-// takes 1.2 - 2 steps.
-struct Lp16Map {
-    uint32_t kmask;     // 2^K - 1
-    uint32_t n_slots;
-    uint32_t magic;     // ceil(2^(K+s) / n_slots), s = ceil(log2 n_slots): exact h / n_slots for h < 2^K
-    uint32_t shift;     // K + s
-    uint32_t tag_bits;  // bits of the largest tag
-    uint32_t dmax;      // largest displacement an entry can record
-};
-
-// true when the id was newly inserted (HashSet::insert); `ovf` is raised when the id would
-// need a displacement beyond dmax
-__device__ __forceinline__ bool lp16_insert(uint32_t* table, const Lp16Map& m, uint32_t id, bool& ovf) {
-    const uint32_t h = (id * 0x9E3779B1u) & m.kmask;
-    const uint32_t tag = (uint32_t)(((uint64_t)h * m.magic) >> m.shift);
-    uint32_t s = h - tag * m.n_slots;
-    uint32_t want = tag;
-    const uint32_t step = 1u << m.tag_bits;
-    for (uint32_t d = 0;;) {
-        uint32_t* wp = table + (s >> 1);
-        const uint32_t w = *wp;
-        const uint32_t cur = (s & 1u) ? (w >> 16) : (w & 0xFFFFu);
-        if (cur == want) return false;
-        if (cur == 0xFFFFu) {
-            const uint32_t neu = (s & 1u) ? ((w & 0xFFFFu) | (want << 16)) : ((w & 0xFFFF0000u) | want);
-            if (atomicCAS(wp, w, neu) == w) return true;
-            continue;  // another lane of this warp changed the word: look at the slot again
-        }
-        if (++d > m.dmax) {
-            ovf = true;
-            return false;
-        }
-        want += step;
-        s = s + 1 == m.n_slots ? 0 : s + 1;
-    }
-}
-
 // Packed f32x2 arithmetic (FADD2 / FFMA2): each half is an IEEE round-to-nearest operation.
 __device__ __forceinline__ uint64_t pack2(float lo, float hi) {
     uint64_t r;
@@ -129,12 +85,8 @@ __device__ __forceinline__ uint4 ldg16(const uint8_t* p) { return __ldg(reinterp
 // All candidate rows of a hop are requested from HBM at once with one bulk L2 prefetch per row
 // (no registers, no shared memory); the register passes below then overlap with the fills and
 // find all but the first rows in L2.
-#ifndef DAB_V3_PREFETCH
-#define DAB_V3_PREFETCH 1  // 0: no bulk L2 prefetch of the candidate rows (tuning)
-#endif
 __device__ __forceinline__ void prefetch_rows(const uint8_t* __restrict__ vectors, size_t row_stride, const uint32_t* __restrict__ cid,
                                               uint32_t n, uint32_t row_bytes16, int lane) {
-    if (!DAB_V3_PREFETCH) return;
     for (uint32_t j = lane; j < n; j += 32) {
         const uint8_t* src = vectors + (size_t)cid[j] * row_stride;
         asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(row_bytes16) : "memory");

@@ -6,10 +6,7 @@
 
 namespace dab {
 
-#ifndef DAB_V2_WARPS
-#define DAB_V2_WARPS 1
-#endif
-constexpr int kV2Warps = DAB_V2_WARPS;  // warps per CTA (each warp owns a query)
+constexpr int kV2Warps = 1;  // warps per CTA (each warp owns a query)
 
 struct SearchParamsV2 {
     const uint8_t* vectors;
@@ -48,7 +45,6 @@ struct SearchParamsV2 {
     uint32_t row_bytes;   // bytes copied per row (multiple of 16)
     uint32_t row_slot;    // bytes between staged rows
     uint32_t stage_rows;  // rows staged per round (multiple of kGroup)
-    unsigned long long* phase_cycles;  // optional [8] per-phase cycle sums (profiling aid)
 };
 
 struct V2Launch {

@@ -33,9 +33,8 @@ struct SearchParamsV3 {
     float* rec_dists;
     uint32_t* rec_counts;
     uint32_t rec_cap;
-    // visited set: 16-bit entries per warp in shared memory (search_smem.cuh): n_buckets buckets of
-    // 16 tags (bucketed variant) or n_buckets * 16 linear-probing slots
-    uint32_t n_buckets, tag_kmask, tag_magic, tag_shift, visited_limit, tag_bits, tag_dmax;
+    // visited set: 16-bit entries per warp in shared memory (search_smem.cuh): n_buckets buckets of 16 tags
+    uint32_t n_buckets, tag_kmask, tag_magic, tag_shift, visited_limit;
     uint32_t fast_nm;  // f32 rows of 32 * fast_nm <= 128 elements: register-resident query, 8 rows per step (0: generic path)
     // per-warp shared memory layout (bytes)
     uint32_t warp_smem, off_q, off_qd, off_qi, off_cid, off_cd, off_beam, off_adj, off_table;

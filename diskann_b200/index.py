@@ -149,10 +149,6 @@ class GpuIndex:
     def set_stream(self, cuda_stream_ptr):
         check(_lib.lib().dab_set_stream(self._h, C.c_void_p(cuda_stream_ptr)))
 
-    def reload_tuning(self):
-        """Re-read the DAB_* tuning knobs from the environment (they are read once at creation otherwise)."""
-        check(_lib.lib().dab_reload_tuning(self._h))
-
     # -- replication (one process per GPU): NCCL inside the library
     @staticmethod
     def comm_unique_id():

@@ -67,11 +67,6 @@ int dab_set_stream(dab_index* idx, void* cuda_stream);
 /* number of kernels this library has launched in this process (bench.py "gpu_launches") */
 uint64_t dab_launch_count(void);
 
-/* The DAB_* tuning / test knobs (csrc/dab_common.cuh, struct Tuning; none changes a result) are read from the
- * environment once, at dab_create.  This re-reads them for an existing handle, so a tuning tool can compare kernel
- * variants on one resident index.  No reference counterpart (tooling only). */
-int dab_reload_tuning(dab_index* idx);
-
 /* ------------------------------------------------------------------ data upload */
 
 /* layers::Set<T>::set(element, bytes) (diskann-inmem/src/layers/mod.rs:79-96) /

@@ -357,9 +357,9 @@ def trained_pq(rng, base, chunks, centers=256):
 @pytest.mark.parametrize("path", ["fused", "separate_kernels"])
 def test_pq_lut_adc_encode_bit_exact(dab, monkeypatch, metric, dim, chunks, path):
     """K6 / K7 through dab_pq_populate_lut / dab_pq_distances: pq_fused_kernel (pivots and the query's table in shared
-    memory, the default where they fit) and the pq_lut_kernel + pq_adc_kernel pair (DAB_PQ_GLOBAL_LUT)."""
+    memory, the default where they fit) and the pq_lut_kernel + pq_adc_kernel pair (DAB_TEST_PQ_GLOBAL_LUT)."""
     if path == "separate_kernels":
-        monkeypatch.setenv("DAB_PQ_GLOBAL_LUT", "1")
+        monkeypatch.setenv("DAB_TEST_PQ_GLOBAL_LUT", "1")
     rng = np.random.default_rng(dim + chunks)
     n, nq, c = 2000, (300 if chunks == 32 else 16), (700 if chunks == 32 else 200)  # > one CTA per SM, > one pass of candidates
     base = clustered(rng, n + 1, dim)
@@ -675,7 +675,7 @@ def test_pq_traversal_search_identical_to_oracle(dab, monkeypatch, dt, metric, d
     lengths 4 / 8 / mixed, 32 / 25 / 16 / 12 / 7 chunks) and search_kernel_pq (per-warp table in global memory),
     and the overflow re-run of the former (a 256-slot visited table)."""
     if path == "global_lut":
-        monkeypatch.setenv("DAB_PQ_GLOBAL_LUT", "1")
+        monkeypatch.setenv("DAB_TEST_PQ_GLOBAL_LUT", "1")
     if path == "smem_pivots_overflow":
         monkeypatch.setenv("DAB_TEST_VISITED_LOG2", "8")
     rng = np.random.default_rng(d + chunks)

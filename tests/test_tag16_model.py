@@ -1,5 +1,5 @@
-"""Host model of the 16-bit quotient-tag visited table prepared for the next round
-(search_common.cuh Tag16Map / tag16_of, built only with -DDAB_V2_TAG16_BUILD=1): the id ->
+"""Host model of the 16-bit quotient-tag visited table (search_common.cuh Tag16Map / tag16_of; the
+shared-memory visited set of search_kernel_v3 and the level-1 table of search_kernel_v2): the id ->
 (bucket, tag) map must be a bijection on [0, 2^K) with 14-bit tags, and the multiply-shift
 division the device uses must be exact."""
 import numpy as np

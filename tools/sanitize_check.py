@@ -29,11 +29,15 @@ if len(sys.argv) > 1 and sys.argv[1] == "pq":
             ids = rng.integers(0, n + 1, (20, 300)).astype(np.uint32)
             lut = g.pq_populate_lut(base[:20].astype(np.float32))
             dd = g.pq_distances(base[:20].astype(np.float32), ids)
-            os.environ["DAB_PQ_GLOBAL_LUT"] = "1"
-            g.reload_tuning()
-            a2 = g.search_batch_pq(base[:48], 5, 40, 1, rerank=True)
-            dd2 = g.pq_distances(base[:20].astype(np.float32), ids)
-            del os.environ["DAB_PQ_GLOBAL_LUT"]
+            # the same index with the per-query tables in global memory (search_kernel_pq, pq_lut_kernel + pq_adc_kernel)
+            os.environ["DAB_TEST_PQ_GLOBAL_LUT"] = "1"
+            with dab.GpuIndex(ddt, dab.Metric.L2, d, n, 1, 41) as g2:
+                g2.upload_vectors(base)
+                g2.upload_graph(adj)
+                g2.upload_pq(*g.download_pq())
+                a2 = g2.search_batch_pq(base[:48], 5, 40, 1, rerank=True)
+                dd2 = g2.pq_distances(base[:20].astype(np.float32), ids)
+            del os.environ["DAB_TEST_PQ_GLOBAL_LUT"]
             assert np.array_equal(a[0], a2[0]) and np.array_equal(dd.view(np.uint32), dd2.view(np.uint32))
             print(dt.__name__, d, chunks, "pq ok", int(a[2].min()), int(b[2].min()), int(c[2].min()), lut.shape)
     for nb in (8, 4, 1):                                                       # MinMax quantizer: compress + distances
